@@ -111,7 +111,7 @@ def test_test_image_matches_oracle(cuda, net_name, C, scales, hw):
     assert e_prob < 1e-4 and e_bbox < 1e-4 and e_rois < 5e-3
 
 
-def test_im_detect_and_fused_detect(cuda):
+def test_im_detect_and_fused_detect(cuda, monkeypatch):
     """im_detect surface + fused post-processing vs the oracle fed with the GPU's own head outputs
     (isolates the tail: decode, clip, per-class NMS, cap -> must be bit-exact)."""
     from model.test import im_detect, detect_image, _detections_python_loop
@@ -121,7 +121,7 @@ def test_im_detect_and_fused_detect(cuda):
     im = rng.integers(0, 256, (240, 320, 3), dtype=np.uint8)
     import cv2
     im = cv2.blur(im, (5, 5))
-    cfg.USE_GPU_NMS = False
+    monkeypatch.setattr(cfg, "USE_GPU_NMS", False)     # restored afterwards: the config is global to the session
     scores, boxes = im_detect(None, net, im)
     blob, scale = P.get_image_blob(im)
     plan = net.plan_for(blob.shape[1], blob.shape[2])

@@ -1,6 +1,5 @@
 """Host-side logic of the reference-facing surface (no GPU): config tree, blobs, anchors, thresholds, imdb,
-tensorflow shim, the N>1 record gather over gloo, and the reference's own tools/demo.py driven unchanged up to the
-(loud) device check."""
+tensorflow shim, the N>1 record gather over gloo, and tools/demo.py driven up to the (loud) device check."""
 import os
 import subprocess
 import sys
@@ -11,7 +10,6 @@ import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 G = np.load(os.path.join(ROOT, "tests", "golden", "reference_vectors.npz"))
-REF = "/root/reference"
 
 
 def test_config_defaults_merge_and_set(tmp_path):
@@ -264,38 +262,25 @@ def test_sharded_test_net_matches_single_process(tmp_path):
                 assert np.array_equal(np.asarray(boxes[j][i], np.float32).reshape(-1, 5), want), (n_images, i, j)
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree only exists in the authoring container")
-def test_reference_demo_script_drives_this_lib_unchanged(tmp_path):
-    """Runs the reference's OWN tools/demo.py (unmodified, in place) against this repo's lib/ + shims.  Without a GPU it
-    must get through argument parsing, cfg, tf.Session, create_architecture, Saver.restore and cv2.imread, and stop at the
-    first image with the loud 'no CUDA device' error -- there is no CPU fallback to fall into."""
+def test_demo_script_stops_loudly_without_a_device(tmp_path):
+    """tools/demo.py with a TensorFlow V2 checkpoint and a directory of images.  Without a GPU it must get through argument
+    parsing, cfg, create_architecture, the strict checkpoint restore and cv2.imread, and stop at the first image with the
+    loud 'no CUDA device' error -- there is no CPU fallback to fall into."""
+    import cv2
     import torch
     if torch.cuda.is_available():
-        pytest.skip("CPU-container check")
-    ck = tmp_path / "output" / "res101" / "voc_2007_trainval+voc_2012_trainval" / "default"
-    ck.mkdir(parents=True)
-    pre = str(ck / "res101_faster_rcnn_iter_110000.ckpt")
+        pytest.skip("checks the behaviour without a CUDA device")
+    pre = str(tmp_path / "res50_faster_rcnn.ckpt")
     subprocess.check_call([sys.executable, os.path.join(ROOT, "tools", "make_synthetic_ckpt.py"), "--net", "res50", "--classes", "21",
-                           "--anchors", "9", "--out", pre], cwd=ROOT)
-    code = textwrap.dedent("""
-        import sys, runpy, types
-        sys.modules["_init_paths"] = types.ModuleType("_init_paths")   # the reference's own file would add ITS lib/ (INTEGRATION.md)
-        sys.path.insert(0, %r)
-        from tf_faster_rcnn_b200 import paths
-        paths.add_lib_path(with_shims=True)
-        from model.config import cfg
-        cfg.DATA_DIR = %r
-        import nets.resnet_v1 as R
-        _orig = R.resnetv1.__init__
-        R.resnetv1.__init__ = lambda self, num_layers=50: _orig(self, 50)   # keep the synthetic checkpoint small
-        sys.argv = ["demo.py", "--net", "res101", "--dataset", "pascal_voc_0712"]
-        runpy.run_path(%r, run_name="__main__")
-    """) % (ROOT, os.path.join(REF, "data"), os.path.join(REF, "tools", "demo.py"))
-    r = subprocess.run([sys.executable, "-c", code], cwd=str(tmp_path), capture_output=True, text=True, timeout=300)
+                           "--anchors", "9", "--format", "bundle", "--out", pre], cwd=ROOT)
+    images = tmp_path / "images"
+    images.mkdir()
+    cv2.imwrite(str(images / "000456.jpg"), np.random.default_rng(0).integers(0, 256, (240, 320, 3), dtype=np.uint8))
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "tools", "demo.py"), "--net", "res50", "--images", str(images),
+                        "--model", pre], cwd=str(tmp_path), capture_output=True, text=True, timeout=300)
     out = r.stdout + r.stderr
     assert r.returncode != 0
-    assert "Loaded network" in out, out[-2000:]
-    assert "Demo for data/demo/000456.jpg" in out, out[-2000:]
+    assert "in im_detect" in out, out[-2000:]
     assert "check_device failed" in out and "no CUDA device" in out, out[-2000:]
 
 
