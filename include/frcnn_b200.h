@@ -88,7 +88,9 @@ int frcnn_nms_sorted_dev(const float* boxes_dev, int n, float thresh, unsigned f
  *                          * scale[co] + shift[co] (+ residual[n,ho,wo,co]) )
  * Requirements: cin % 32 == 0.  w_hi/w_lo from frcnn_pack_conv_weights.  scale may be NULL (=1). */
 typedef struct frcnn_conv_plan frcnn_conv_plan;
-#define FRCNN_CONV_F16X3 0   /* fp16 hi/lo split of both operands, 3 x tcgen05.mma.kind::f16, fp32 accumulate */
+#define FRCNN_CONV_F16X3 0   /* fp16 hi/lo split of both operands, 3 x tcgen05.mma.kind::f16, fp32 accumulate.  Activation range:
+                              * fp32-grade for |x| < 65520; an activation of larger magnitude (like an Inf or NaN) makes every
+                              * output whose window reads it Inf or NaN, and leaves all other outputs unaffected. */
 #define FRCNN_CONV_TF32X3 1  /* tf32 hi/lo split, 3 x kind::tf32 (same 22-bit products, twice the tensor time) */
 #define FRCNN_CONV_F16X1 2   /* THROUGHPUT mode, not fp32-grade: plain fp16 operands (the hi planes only), 1 MMA per product, fp32
                               * accumulate; ~3e-4 of the output range per layer instead of ~4e-7.  Same packed weights as F16X3. */

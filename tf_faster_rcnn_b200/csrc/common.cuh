@@ -186,10 +186,11 @@ __device__ __forceinline__ void mbar_wait2(uint32_t bar0, uint32_t par0, uint32_
 // register re-allocation between warp roles: every warp of a warpgroup (4 consecutive warps) executes the same one
 template <int R> __device__ __forceinline__ void reg_dec() { asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(R)); }
 template <int R> __device__ __forceinline__ void reg_inc() { asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(R)); }
-// two fp32 -> packed fp16x2 (lo half = a, hi half = b), round to nearest even, saturating to +-65504
-__device__ __forceinline__ uint32_t pack_f16x2_sat(float a, float b) {
+// two fp32 -> packed fp16x2 (lo half = a, hi half = b), round to nearest even, IEEE overflow: |x| >= 65520 becomes +-Inf and
+// NaN stays NaN (no .satfinite: a saturated operand would turn an out-of-range activation into a finite, wrong product)
+__device__ __forceinline__ uint32_t pack_f16x2_rn(float a, float b) {
   uint32_t r;
-  asm("cvt.rn.satfinite.f16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(b), "f"(a));
+  asm("cvt.rn.f16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(b), "f"(a));
   return r;
 }
 // one lane of a converged warp (the rest of the warp stays converged: operands remain in uniform registers)

@@ -545,8 +545,10 @@ conv_gemm_tf32x3_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_co
 //       to 2^-22 relative exactly like the tf32 hi/lo pair, at half the tensor time and half the B bytes (shared memory,
 //       L2).  Range: the lo planes are pre-scaled by 2^11 (D_small is folded back with one fma by 2^-11), weights are
 //       pre-scaled per layer by a power of two so that max|w| sits in [2^13, 2^14) (undone exactly by `out_mult` in the
-//       epilogue), activations are converted with saturation (|x| <= 65504; anything the nets here produce is orders of
-//       magnitude below).  Tiny values lose nothing: |x| < 2^-14 still resolves to 2^-35 absolute through the lo plane.
+//       epilogue).  Activations are converted with round-to-nearest and IEEE overflow: fp32-grade for |x| < 65520 (then
+//       |x - x_hi| <= 16, so the lo plane stays in range), while a larger |x|, Inf or NaN turns every output it feeds into
+//       Inf / NaN, as fp32 arithmetic would -- never into a finite wrong value.  Tiny values lose little: an activation
+//       below fp16's normal range (|x| < 2^-14) keeps 2^-36 absolute through the subnormal lo plane.
 //   (2) r01's operand splitter was issue bound: ONE warp per TMEM lane quarter, 334 instructions per k-block at the 0.5 IPC a
 //       single warp gets from the fma/alu pipes.  Now 8 splitter warps (group g converts the g-th 32-channel half of every
 //       64-wide k-block), 4 instructions per element on packed pairs, and A / B have their own producer warps and rings.
@@ -667,13 +669,13 @@ conv_gemm_f16x3_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_con
 #pragma unroll
         for (int c = 0; c < 8; ++c) {
           const float4 v = lds_f4(coff[c] + stage_off);
-          const uint32_t h01 = pack_f16x2_sat(v.x, v.y), h23 = pack_f16x2_sat(v.z, v.w);
+          const uint32_t h01 = pack_f16x2_rn(v.x, v.y), h23 = pack_f16x2_rn(v.z, v.w);
           const float2 f01 = __half22float2(*reinterpret_cast<const __half2*>(&h01));
           const float2 f23 = __half22float2(*reinterpret_cast<const __half2*>(&h23));
           pk[2 * c] = h01; pk[2 * c + 1] = h23;
           if (!X1) {
-            pk[16 + 2 * c] = pack_f16x2_sat(__fmul_rn(__fsub_rn(v.x, f01.x), 2048.f), __fmul_rn(__fsub_rn(v.y, f01.y), 2048.f));
-            pk[16 + 2 * c + 1] = pack_f16x2_sat(__fmul_rn(__fsub_rn(v.z, f23.x), 2048.f), __fmul_rn(__fsub_rn(v.w, f23.y), 2048.f));
+            pk[16 + 2 * c] = pack_f16x2_rn(__fmul_rn(__fsub_rn(v.x, f01.x), 2048.f), __fmul_rn(__fsub_rn(v.y, f01.y), 2048.f));
+            pk[16 + 2 * c + 1] = pack_f16x2_rn(__fmul_rn(__fsub_rn(v.z, f23.x), 2048.f), __fmul_rn(__fsub_rn(v.w, f23.y), 2048.f));
           } else {
             pk[16 + 2 * c] = 0u; pk[16 + 2 * c + 1] = 0u;
           }
